@@ -17,6 +17,9 @@ One "step" = one full ICRL learner iteration on synthetic buffers of the named e
 `cpu_baseline`: the UNMODIFIED reference (baseline/_ref) on a bounded sample of the same iteration, extrapolated linearly
            (the oracle port only if that copy is absent).
 Fixed work: KL early stops (ppo target_kl, cn target_kl_*) are disabled so every epoch / backward iteration runs.
+`--dump-outputs DIR`: what the last timed step computed, as DIR/<name>.npy (see dump_outputs).  The inputs depend only on
+the arguments, so two builds run with the same arguments can be compared array by array.  Inside the tree, use
+`bench_outputs/` (git-ignored).
 """
 import argparse
 import json
@@ -57,6 +60,9 @@ def parse():
     ap.add_argument("--aux-steps", type=int, default=2, help="timed iterations of each secondary workload")
     ap.add_argument("--no-sweep", action="store_true", help="skip the Ant-shaped 64K-16M transition sweep")
     ap.add_argument("--sweep-sizes", default="65536,262144,1048576,4194304,16777216", help="transitions per GPU")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the main workload computed as DIR/<name>.npy (rank 0); "
+                         "bench_outputs/ in the repository root is git-ignored for this")
     return ap.parse_args()
 
 
@@ -685,8 +691,37 @@ def ant_sweep(rank, world, dev, ppo_comm, peaks, sizes):
     return rows_out
 
 
-def run_workload(name, args, rank, world, local, ppo_comm, peaks, flush, steps, warmup, want_e2e, want_family):
-    """value (device-resident DeviceLearner), e2e (host-buffer public API) and the K4 launch roofline of one named workload."""
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(learner, out_dir):
+    """What the last DeviceLearner.run() computed, as out_dir/<name>.npy: per rollout the K1 costs (and their K5
+    normalisation), K3 advantages and returns and K4 per-optimiser-step statistics; the policy, constraint net, Adam
+    moments, dual variable and cost statistics the iteration leaves behind; the K2 metrics.  float32, or float64 where the
+    path keeps float64.  Must run before anything else touches the learner: the e2e leg trains the same constraint net and
+    the roofline relaunches K4."""
+    w, pol, cn = learner.w, learner.policy, learner.cn
+    arrays = {"costs": learner.costs, "reward_advantages": learner.adv_r, "reward_returns": learner.ret_r,
+              "cost_advantages": learner.adv_c, "cost_returns": learner.ret_c, "ppo_step_stats": learner.stats,
+              "policy_params": pol._params, "policy_adam_m": pol._adam_m, "policy_adam_v": pol._adam_v,
+              "dual_state": learner.dual.nu.state, "cn_params": cn._params, "cn_adam_m": cn._adam_m, "cn_adam_v": cn._adam_v}
+    if w.normalize_cost:
+        arrays.update(normalized_costs=learner.costs_norm, cost_norm_state=learner.cost_state)
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    if w.backward_iters > 0 and w.nominal_rows > 0:
+        m = learner.last_cn_metrics
+        arrays["cn_train_metrics"] = np.array([getattr(m, f) for f, _ in m._fields_], np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (k, a.dtype)
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
+def run_workload(name, args, rank, world, local, ppo_comm, peaks, flush, steps, warmup, want_e2e, want_family, dump_dir=None):
+    """value (device-resident DeviceLearner), e2e (host-buffer public API) and the K4 launch roofline of one named workload;
+    with `dump_dir`, rank 0 also writes what the last timed step computed (dump_outputs)."""
     from icrl_b200 import _lib
     from icrl_b200.learner import WORKLOADS, DeviceLearner
     w = WORKLOADS[name]
@@ -705,6 +740,8 @@ def run_workload(name, args, rank, world, local, ppo_comm, peaks, flush, steps, 
     launches = _lib.lib().icrl_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
     learner.check()                                   # raises on an exchange time-out (result[2]) in any K4 launch
+    if dump_dir is not None and rank == 0:
+        dump_outputs(learner, dump_dir)
     per_step = t_dev / steps
     total_tr = w.transitions_per_iteration * world
     out = {"workload": w.name, "value": total_tr / per_step, "unit": UNIT, "ms_per_step": per_step * 1e3, "steps": steps,
@@ -813,7 +850,7 @@ def main():
             raise SystemExit(f"data-parallel parity FAILED, nothing timed: {dp_parity}")
     flush = th.zeros(64 * 1024 * 1024, device="cuda")      # 256 MB
     main_out, learner = run_workload(args.workload, args, rank, world, local, ppo_comm, peaks, flush, args.steps, args.warmup,
-                                     not args.no_e2e, True)
+                                     not args.no_e2e, True, dump_dir=args.dump_outputs)
     del learner
     th.cuda.empty_cache()
     # the other BASELINE configs, short runs (N>1: AntWall only -- BASELINE config 3 is "AntWall on 1/2/4/8 B200")
