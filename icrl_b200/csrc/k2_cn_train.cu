@@ -472,7 +472,7 @@ __global__ void __launch_bounds__(128) cn_grad_kernel(const __grid_constant__ Cn
                     const float l1 = fmaxf(logf(1.f - pr), -100.f);            // nn.BCELoss clamps log at -100
                     st[ST_NLOG] += logf(pr + eps);      // `unweighted_nominal_loss` is mean(log(p + eps)) in both modes (:211)
                     st[ST_NWLOG] += -l1;                // BCE(p, 0)
-                    dLdp = (l1 > -100.f ? 1.f / (1.f - pr) : 0.f) * inv_nn;
+                    dLdp = pr / fmaxf((1.f - pr) * pr, 1e-12f) * inv_nn;           // BCELoss backward, y = 0
                 } else {
                     const float lg = logf(pr + eps);
                     st[ST_NLOG] += lg; st[ST_NWLOG] += wi * lg;
@@ -484,7 +484,9 @@ __global__ void __launch_bounds__(128) cn_grad_kernel(const __grid_constant__ Cn
                 if (gail) {
                     const float l1 = fmaxf(logf(pr), -100.f);
                     st[ST_ELOG] += -l1;
-                    dLdp = (l1 > -100.f ? -1.f / pr : 0.f) * inv_ne;
+                    // BCELoss backward with y = 1: (p - 1) / max((1 - p) p, 1e-12), so the gradient fades out on rows the
+                    // discriminator rejects with p < 1e-12 instead of pushing them at full strength (-1 / p)
+                    dLdp = (pr - 1.f) / fmaxf((1.f - pr) * pr, 1e-12f) * inv_ne;
                 } else {
                     st[ST_ELOG] += logf(pr + eps);
                     dLdp = -inv_ne / (pr + eps) - reg * inv_ne;

@@ -162,6 +162,30 @@ def batches(batch_size, nom_size, exp_size):
         yield indices[start:start + batch_size], indices[start:start + batch_size]
 
 
+def loss_terms(spec: CNSpec, nominal_preds: th.Tensor, expert_preds: th.Tensor, is_batch: th.Tensor,
+               materialize_broadcast: bool = False):
+    """constraint_net.py:193-202: (loss, nominal_loss, expert_loss, regularizer_loss) of one batch.  Works in the dtype
+    of the predictions, so a float64 forward gives the float64 loss (and, through autograd, the float64 gradient).
+    `is_batch` is the weight tensor as `train` shapes it: [N,1,1] in per-step IS mode (quirk A), [N,1] otherwise."""
+    eps = spec.eps
+    if spec.train_gail_lambda:                                    # :193-197
+        bce = th.nn.BCELoss()
+        nominal_loss = bce(nominal_preds, th.zeros(*nominal_preds.size(), dtype=nominal_preds.dtype))
+        expert_loss = bce(expert_preds, th.ones(*expert_preds.size(), dtype=expert_preds.dtype))
+        regularizer_loss = th.tensor(0)
+        loss = nominal_loss + expert_loss
+    else:                                                         # :199-202
+        expert_loss = th.mean(th.log(expert_preds + eps))
+        log_nom = th.log(nominal_preds + eps)
+        if is_batch.dim() == 3 and not materialize_broadcast:
+            nominal_loss = th.mean(is_batch) * th.mean(log_nom)
+        else:
+            nominal_loss = th.mean(is_batch * log_nom)
+        regularizer_loss = spec.regularizer_coeff * (th.mean(1 - expert_preds) + th.mean(1 - nominal_preds))
+        loss = (-expert_loss + nominal_loss) + regularizer_loss
+    return loss, nominal_loss, expert_loss, regularizer_loss
+
+
 def train(params, adam_state, spec: CNSpec, iterations: int, nominal_obs, nominal_acs, episode_lengths,
           expert_obs, expert_acs, lr: float, adam_eps: float = 1e-5, materialize_broadcast: bool = False,
           batch_size: Optional[int] = None):
@@ -204,21 +228,8 @@ def train(params, adam_state, spec: CNSpec, iterations: int, nominal_obs, nomina
             is_batch = (is_weights if nom_idx is None else is_weights[nom_idx])[..., None]
             nominal_preds = forward(params, nominal_batch)
             expert_preds = forward(params, expert_batch)
-            if spec.train_gail_lambda:                                    # :193-197
-                bce = th.nn.BCELoss()
-                nominal_loss = bce(nominal_preds, th.zeros(*nominal_preds.size()))
-                expert_loss = bce(expert_preds, th.ones(*expert_preds.size()))
-                regularizer_loss = th.tensor(0)
-                loss = nominal_loss + expert_loss
-            else:                                                         # :199-202
-                expert_loss = th.mean(th.log(expert_preds + eps))
-                log_nom = th.log(nominal_preds + eps)
-                if is_batch.dim() == 3 and not materialize_broadcast:
-                    nominal_loss = th.mean(is_batch) * th.mean(log_nom)
-                else:
-                    nominal_loss = th.mean(is_batch * log_nom)
-                regularizer_loss = spec.regularizer_coeff * (th.mean(1 - expert_preds) + th.mean(1 - nominal_preds))
-                loss = (-expert_loss + nominal_loss) + regularizer_loss
+            loss, nominal_loss, expert_loss, regularizer_loss = loss_terms(spec, nominal_preds, expert_preds, is_batch,
+                                                                           materialize_broadcast)
             grads = th.autograd.grad(loss, params)
             adam_step(params, grads, adam_state, lr, eps=adam_eps)
 

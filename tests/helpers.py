@@ -58,6 +58,35 @@ def max_param_err(pa, pb):
     return worst
 
 
+def cn_grad64(params, spec, nominal_obs, nominal_acs, episode_lengths, expert_obs, expert_acs, start_params=None):
+    """The float64 gradient of the K2 loss (ocn.loss_terms, full batch) at `params`, as a list of float64 arrays in the
+    order of `params`.  The inputs are prepared in float32 as the reference prepares them, then widened; with importance
+    sampling the weights come from float64 predictions at `start_params` (default: `params`, i.e. iteration 0) and at
+    `params`."""
+    p64 = [th.as_tensor(np.asarray(p), dtype=th.float64).clone().requires_grad_(True) for p in params]
+    xn = th.tensor(ocn.prepare_data(spec, nominal_obs, nominal_acs), dtype=th.float64)
+    xe = th.tensor(ocn.prepare_data(spec, expert_obs, expert_acs), dtype=th.float64)
+    if spec.importance_sampling:
+        s64 = p64 if start_params is None else [th.as_tensor(np.asarray(p), dtype=th.float64) for p in start_params]
+        with th.no_grad():
+            old, new = ocn.forward(s64, xn), ocn.forward(p64, xn)
+        w, _, _ = ocn.compute_is_weights(old, new, episode_lengths, spec.eps, spec.per_step_importance_sampling)
+        w = w.to(th.float64)
+    else:
+        w = th.ones(xn.shape[0], dtype=th.float64)
+    loss = ocn.loss_terms(spec, ocn.forward(p64, xn), ocn.forward(p64, xe), w[..., None])[0]
+    return [g.numpy() for g in th.autograd.grad(loss, p64)]
+
+
+def max_grad_err(got, want):
+    """max over tensors of ||got-want||_inf / ||want||_inf (a tensor whose reference gradient is all zero must be zero)."""
+    worst = 0.0
+    for a, b in zip(got, want):
+        a, b = np.asarray(a, np.float64), np.asarray(b, np.float64)
+        worst = max(worst, float(np.max(np.abs(a - b)) / max(float(np.max(np.abs(b))), 1e-30)))
+    return worst
+
+
 def k4x_inputs(seed, T, E, obs_dim, acs_dim, is_discrete):
     """The seeded inputs of the round-2 K4 fixtures (tests/golden/make_golden.py::k4x_inputs, same generator calls in the
     same order): only torch-dependent arrays and outputs are stored in the .npz files."""

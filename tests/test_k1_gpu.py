@@ -11,9 +11,9 @@ from oracle import cn as ocn
 pytestmark = pytest.mark.gpu
 
 
-def make_cn(shape, d, **kw):
+def make_cn(shape, d, hidden=None, **kw):
     from icrl_b200.constraint_net import ConstraintNet
-    s = SHAPES[shape]
+    s = dict(SHAPES[shape], **({"hidden": hidden} if hidden else {}))
     low = high = None
     if not s["is_discrete"]:
         low, high = -np.ones(s["acs_dim"], np.float32), np.ones(s["acs_dim"], np.float32)
@@ -72,17 +72,45 @@ def test_load_frozen_checkpoint(tmp_path, name, kw):
     assert_cost_close(cn.cost_function(d["obs"], d["acs"]), d["cost"])
 
 
-@pytest.mark.parametrize("n", [1, 5, 31, 127, 128, 129, 1000, 4096 + 17])
-@pytest.mark.parametrize("shape", ["lgw", "ant"])
+# synthetic nets "<inputs>_<hidden widths>_<observation dtype>": every padded width the kernels are built for (8 16 24 32
+# 40 48 64), one to three hidden layers, a narrower layer after a wider one, float32 and float64 observations
+SYNTH_NETS = ["hc_5_f64", "hc_16x16x16_f32", "ant_32x32_f64", "ant_48x7_f32", "hc_20_f64", "ant_40x40_f64",
+              "hc_64x64_f32", "lgw_64x64_f64", "ant_64x64_f32", "ant_64x64_f64", "hc_64x64x64_f32", "hc_64x64x64_f64"]
+
+
+def synthetic_net(name):
+    """A golden-shaped dict for a synthetic net: weights uniform in +-1/sqrt(fan_in) (nn.Linear's default range) under a
+    fixed seed, observation normalisation to unit scale for the `* 6` observations of the ragged test."""
+    shape, widths, tag = name.split("_")
+    hidden = tuple(int(w) for w in widths.split("x"))
+    s = dict(SHAPES[shape], hidden=hidden)
+    g = th.Generator().manual_seed(len(hidden) * 100 + sum(hidden))
+    dims = [s["obs_dim"] + s["acs_dim"]] + list(hidden) + [1]
+    d = {"obs_mean": np.zeros(s["obs_dim"]), "obs_var": np.full(s["obs_dim"], 36.0)}
+    for i in range(len(dims) - 1):
+        bound = 1.0 / np.sqrt(dims[i])
+        d[f"p.{2 * i}.weight"] = ((th.rand(dims[i + 1], dims[i], generator=g) * 2 - 1) * bound).numpy()
+        d[f"p.{2 * i}.bias"] = ((th.rand(dims[i + 1], generator=g) * 2 - 1) * bound).numpy()
+    return shape, s, d, np.float64 if tag == "f64" else np.float32
+
+
+@pytest.mark.parametrize("n", [1, 5, 31, 127, 128, 129, 1000, 4096 + 17, 16, 17, 18_949, 100_003])
+@pytest.mark.parametrize("shape", ["lgw", "ant"] + SYNTH_NETS)
 def test_ragged_sizes_vs_oracle(shape, n):
-    d = load_golden(f"k1_{shape}_norm_f32")
-    s = SHAPES[shape]
+    """Row counts around the tile and warp sizes, and past 128 x 148 (18 949: the packed kernel is the default there for
+    nets up to 32 wide), on the golden nets and on synthetic nets of every width."""
+    if shape in SHAPES:
+        s, d, dtype = SHAPES[shape], load_golden(f"k1_{shape}_norm_f32"), np.float32
+        cn = make_cn(shape, d)
+    else:
+        shape, s, d, dtype = synthetic_net(shape)
+        cn = make_cn(shape, d, hidden=s["hidden"])
     rng = np.random.default_rng(n)
-    obs = (rng.standard_normal((n, s["obs_dim"])) * 6).astype(np.float32)
+    obs = (rng.standard_normal((n, s["obs_dim"])) * 6).astype(dtype)
     acs = (rng.integers(0, s["acs_dim"], (n, 1)).astype(np.float32) if s["is_discrete"]
            else rng.standard_normal((n, s["acs_dim"])).astype(np.float32) * 1.5)
-    want = ocn.cost_function(cn_params(d), cn_spec(shape, d), obs, acs)
-    assert_cost_close(make_cn(shape, d).cost_function(obs, acs), want)
+    want = ocn.cost_function(cn_params(d), cn_spec(shape, d, hidden_sizes=s["hidden"]), obs, acs)
+    assert_cost_close(cn.cost_function(obs, acs), want)
 
 
 def test_empty_batch():

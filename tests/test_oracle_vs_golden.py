@@ -85,6 +85,26 @@ def test_k2_train_matches_reference(case):
         assert adam["step"] == nstep
 
 
+@pytest.mark.parametrize("case", [c for c in K2_CASES if c.startswith("hc_") or "gail" in c])
+def test_k2_float64_gradient_matches_first_adam_moment(case):
+    """Adam's first moment after one step is exactly (1 - beta1) * g, so the fp32 oracle's exp_avg after one full-batch
+    iteration reads back its gradient: the float64 gradient of ocn.loss_terms (the GPU suite's chain-free reference) must
+    equal it to fp32 rounding.  Measured worst, relative to the tensor's largest entry: 7.9e-6 on the output bias (whose
+    gradient is a difference of the nominal and the expert sums), <= 1.3e-6 on every other tensor."""
+    from helpers import cn_grad64, max_grad_err
+    d = load_golden(f"k2_{case}")
+    spec = cn_spec(case.split("_")[0], d, regularizer_coeff=float(d["reg"]), importance_sampling=not bool(d["no_is"]),
+                   per_step_importance_sampling=bool(d["per_step"]), train_gail_lambda=bool(d.get("gail", False)))
+    params = cn_params(d, "p0.")
+    g64 = cn_grad64(params, spec, d["nominal_obs"], d["nominal_acs"], d["lengths"], d["expert_obs"], d["expert_acs"])
+    adam = ocn.adam_init(params)
+    ocn.train(params, adam, spec, 1, d["nominal_obs"], d["nominal_acs"], d["lengths"], d["expert_obs"], d["expert_acs"],
+              lr=float(d["lr"]))
+    assert adam["step"] == 1
+    err = max_grad_err([m.numpy() for m in adam["exp_avg"]], [0.1 * g for g in g64])
+    assert err <= 2e-5, err
+
+
 @pytest.mark.parametrize("case", ["hc_perstep_mild", "ant_perstep"])
 def test_k2_quirk_a_identity(case):
     """mean over the reference's [N,N,1] broadcast == mean(w) * mean(log p): the O(N) form the product uses."""
