@@ -155,7 +155,7 @@ def train(P, adam_state, flat, perms, *, is_discrete, batch_size, n_epochs, lr, 
     n = flat["observations"].shape[0]
     bs = n if batch_size is None else batch_size
     per_step = {k: [] for k in ("pg_loss", "clip_fraction", "reward_value_loss", "cost_value_loss", "entropy_loss",
-                                "loss", "approx_kl")}
+                                "loss", "approx_kl", "grad_norm")}      # grad_norm: clip_grad_norm_'s pre-clip total norm
     all_kl, early_stop_epoch, steps = [], n_epochs, 0
     done = False
     for epoch in range(n_epochs):
@@ -170,10 +170,11 @@ def train(P, adam_state, flat, perms, *, is_discrete, batch_size, n_epochs, lr, 
                                       clip_range_reward_vf, clip_range_cost_vf)
             grads = th.autograd.grad(loss, params, allow_unused=True)
             grads = [th.zeros_like(p) if g is None else g for p, g in zip(params, grads)]
-            grads, _ = clip_grad_norm(grads, max_grad_norm)
+            grads, total = clip_grad_norm(grads, max_grad_norm)
             adam_step(params, grads, adam_state, lr, eps=adam_eps)
-            for k in per_step:
+            for k in st:
                 per_step[k].append(st[k])
+            per_step["grad_norm"].append(float(total))
             kls.append(st["approx_kl"])
             steps += 1
             if max_steps is not None and steps >= max_steps:

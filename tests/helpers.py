@@ -87,6 +87,23 @@ def max_grad_err(got, want):
     return worst
 
 
+class FakeVecEnv:
+    """Just enough of a VecEnv to build a PPOLagrangian whose rollout buffer the test fills by hand."""
+
+    def __init__(self, obs_dim, act_dim, discrete, n_envs):
+        from icrl_b200.spaces import Box, Discrete
+        self.observation_space = Box(-np.inf, np.inf, (obs_dim,), np.float32)
+        self.action_space = Discrete(act_dim) if discrete else Box(-1, 1, (act_dim,), np.float32)
+        self.num_envs = n_envs
+
+    def reset(self):
+        return np.zeros((self.num_envs,) + self.observation_space.shape, np.float32)
+
+    def step(self, actions):
+        n = self.num_envs
+        return self.reset(), np.zeros(n, np.float32), np.zeros(n, bool), [{} for _ in range(n)]
+
+
 def k4x_inputs(seed, T, E, obs_dim, acs_dim, is_discrete):
     """The seeded inputs of the round-2 K4 fixtures (tests/golden/make_golden.py::k4x_inputs, same generator calls in the
     same order): only torch-dependent arrays and outputs are stored in the .npz files."""

@@ -8,25 +8,10 @@ import pytest
 import torch as th
 
 from conftest import GOLDEN, load_golden
-from helpers import PARAM_RTOL, max_param_err
+from helpers import PARAM_RTOL, FakeVecEnv, max_param_err
 
 pytestmark = pytest.mark.gpu
 K4_CASES = sorted(os.path.basename(p)[3:-4] for p in glob.glob(os.path.join(GOLDEN, "k4_*.npz")))
-
-
-class FakeVecEnv:
-    def __init__(self, obs_dim, act_dim, discrete, n_envs):
-        from icrl_b200.spaces import Box, Discrete
-        self.observation_space = Box(-np.inf, np.inf, (obs_dim,), np.float32)
-        self.action_space = Discrete(act_dim) if discrete else Box(-1, 1, (act_dim,), np.float32)
-        self.num_envs = n_envs
-
-    def reset(self):
-        return np.zeros((self.num_envs,) + self.observation_space.shape, np.float32)
-
-    def step(self, actions):
-        n = self.num_envs
-        return self.reset(), np.zeros(n, np.float32), np.zeros(n, bool), [{} for _ in range(n)]
 
 
 def build_algo(d):

@@ -208,6 +208,30 @@ def test_k4_train_matches_reference(case):
                 assert abs(v - log[k]) <= 1e-5 * max(abs(log[k]), 1e-2), (k, v, log[k])
 
 
+def test_k4_float64_gradient_matches_reference_first_adam_moment():
+    """k4_hc_fullbatch takes one full-batch optimiser step, after which the reference's exp_avg is exactly
+    (1 - beta1) * (clipped gradient): the float64 gradient of oracle.ppo.minibatch_loss at p0, clipped the torch way (the
+    GPU sweep's chain-free reference, tests/test_k4_sweep_gpu.py), must equal it to fp32 rounding.  Measured worst,
+    per tensor relative to its largest entry: 1.1e-6."""
+    from helpers import max_grad_err
+    d = load_golden("k4_hc_fullbatch")
+    flat, hp = k4_inputs(d)
+    names = [str(n) for n in d["param_order"]]
+    P = {n: th.tensor(d["p0." + n], dtype=th.float64, requires_grad=True) for n in names}
+    mb = {k: th.tensor(v, dtype=th.float64) for k, v in flat.items()}
+    for k in oppo.FLAT_FIELDS[2:]:
+        mb[k] = mb[k].flatten()
+    nu = float(oppo.dual_nu(oppo.dual_init(hp["penalty_initial_value"])))
+    opt = lambda k: None if hp[k] < 0 else hp[k]
+    loss, _ = oppo.minibatch_loss(P, mb, "log_std" not in names, hp["clip_range"], nu, hp["ent_coef"], 0.5, 0.5,
+                                  opt("clip_range_reward_vf"), opt("clip_range_cost_vf"))
+    g, _ = oppo.clip_grad_norm(th.autograd.grad(loss, list(P.values())), hp.get("max_grad_norm", 0.5))
+    want = [d[f"adam.{i}.exp_avg"].astype(np.float64) / (1 - 0.9) for i in range(len(names))]
+    assert hp["batch_size"] < 0 or int(hp["batch_size"]) >= flat["observations"].shape[0]
+    err = max_grad_err([x.numpy() for x in g], want)
+    assert err <= 1e-5, err
+
+
 # ------------------------------------------------------------------------------------------- cost normalisation (f1)
 @pytest.mark.parametrize("name,norm", [("all", True), ("nocost", False)])
 def test_costnorm_oracle_matches_reference_wrappers(name, norm):
