@@ -27,7 +27,8 @@ __host__ __device__ inline int ppo_ldx(int D) {
 }
 
 struct PpoArgs {
-    int D, DP, KP, A, is_discrete, h0, h1;
+    int D, DP, KP, A, is_discrete;
+    int h0[3], h1[3];             // hidden widths of the pi, vf and cvf trunks (every tile is padded to H = 64 regardless)
     int T, E, N, B, n_epochs, steps_per_epoch, max_steps;
     int has_target_kl, has_clip_vf_r, has_clip_vf_c;
     float clip_range, clip_vf_r, clip_vf_c, ent_coef, vf_coef_r, vf_coef_c, max_grad_norm, nu;
@@ -72,14 +73,15 @@ inline int ppo_fill_offsets(PpoArgs& a) {
     a.off_logstd = a.is_discrete ? -1 : 0;
     if (!a.is_discrete) o += a.A;
     for (int t = 0; t < 3; ++t) {
-        a.off_w1[t] = o; o += a.h0 * a.D;
-        a.off_b1[t] = o; o += a.h0;
-        a.off_w2[t] = o; o += a.h1 * a.h0;
-        a.off_b2[t] = o; o += a.h1;
+        const int h0 = a.h0[t], h1 = a.h1[t];
+        a.off_w1[t] = o; o += h0 * a.D;
+        a.off_b1[t] = o; o += h0;
+        a.off_w2[t] = o; o += h1 * h0;
+        a.off_b2[t] = o; o += h1;
     }
     const int outs[3] = {a.A, 1, 1};
     for (int t = 0; t < 3; ++t) {
-        a.off_hw[t] = o; o += outs[t] * a.h1;
+        a.off_hw[t] = o; o += outs[t] * a.h1[t];
         a.off_hb[t] = o; o += outs[t];
     }
     return o;
@@ -89,11 +91,25 @@ inline int ppo_make_args(const icrl_ppo_cfg* c, PpoArgs& a) {
     ICRL_CHECK_ARG(c != nullptr, "ppo cfg is NULL");
     ICRL_CHECK_ARG(c->obs_dim >= 1, "obs_dim must be >= 1");
     ICRL_CHECK_ARG(c->act_dim >= 1 && c->act_dim <= AMAX, "act_dim %d out of range (1..%d)", c->act_dim, AMAX);
-    ICRL_CHECK_ARG(c->hidden[0] >= 1 && c->hidden[0] <= H && c->hidden[1] >= 1 && c->hidden[1] <= H,
-                   "policy hidden sizes (%d, %d) must be in 1..%d (two hidden layers per trunk)", c->hidden[0],
-                   c->hidden[1], H);
+    bool per_trunk = false;
+    for (int t = 0; t < 3; ++t) per_trunk |= c->trunk_hidden[t][0] != 0 || c->trunk_hidden[t][1] != 0;
+    if (per_trunk) {
+        static const char* const names[3] = {"pi", "vf", "cvf"};
+        for (int t = 0; t < 3; ++t)
+            ICRL_CHECK_ARG(c->trunk_hidden[t][0] >= 1 && c->trunk_hidden[t][0] <= H && c->trunk_hidden[t][1] >= 1 &&
+                               c->trunk_hidden[t][1] <= H,
+                           "trunk_hidden[%d] (%s) = (%d, %d): both widths must be in 1..%d (two hidden layers per trunk)", t,
+                           names[t], c->trunk_hidden[t][0], c->trunk_hidden[t][1], H);
+    } else {
+        ICRL_CHECK_ARG(c->hidden[0] >= 1 && c->hidden[0] <= H && c->hidden[1] >= 1 && c->hidden[1] <= H,
+                       "policy hidden sizes (%d, %d) must be in 1..%d (two hidden layers per trunk)", c->hidden[0],
+                       c->hidden[1], H);
+    }
     a.D = c->obs_dim; a.DP = ppo_ldx(c->obs_dim); a.KP = ppo_kp(c->obs_dim); a.A = c->act_dim; a.is_discrete = c->is_discrete;
-    a.h0 = c->hidden[0]; a.h1 = c->hidden[1];
+    for (int t = 0; t < 3; ++t) {
+        a.h0[t] = per_trunk ? c->trunk_hidden[t][0] : c->hidden[0];
+        a.h1[t] = per_trunk ? c->trunk_hidden[t][1] : c->hidden[1];
+    }
     a.T = c->T; a.E = c->E; a.N = c->T * c->E;
     a.B = c->batch_size > 0 ? c->batch_size : a.N;
     if (a.B > a.N && a.N > 0) a.B = a.N;

@@ -64,23 +64,24 @@ __global__ void __launch_bounds__(NTH) policy_forward_kernel(const __grid_consta
     const FwdSmem L = fwd_smem_layout(DP);
     const int tid = threadIdx.x, trunk = blockIdx.y, D = a.D;
     const int AOUT = trunk == 0 ? a.A : 1;
+    const int h0 = a.h0[trunk], h1 = a.h1[trunk];
     float* W1t = sm + L.w1t; float* W2t = sm + L.w2t; float* B1 = sm + L.b1; float* B2 = sm + L.b2;
     float* HW = sm + L.hw; float* HB = sm + L.hb; float* X = sm + L.x; float* H1 = sm + L.h1; float* H2 = sm + L.h2;
     for (int i = tid; i < DP * H; i += NTH) {
         const int k = i / H, j = i - k * H;
-        W1t[i] = (k < D && j < a.h0) ? a.params[a.off_w1[trunk] + j * D + k] : 0.f;
+        W1t[i] = (k < D && j < h0) ? a.params[a.off_w1[trunk] + j * D + k] : 0.f;
     }
     for (int i = tid; i < H * H; i += NTH) {
         const int k = i / H, j = i - k * H;
-        W2t[i] = (k < a.h0 && j < a.h1) ? a.params[a.off_w2[trunk] + j * a.h0 + k] : 0.f;
+        W2t[i] = (k < h0 && j < h1) ? a.params[a.off_w2[trunk] + j * h0 + k] : 0.f;
     }
     for (int i = tid; i < AMAX * WA_LD; i += NTH) {
         const int d = i / WA_LD, k = i - d * WA_LD;
-        HW[i] = (d < AOUT && k < a.h1) ? a.params[a.off_hw[trunk] + d * a.h1 + k] : 0.f;
+        HW[i] = (d < AOUT && k < h1) ? a.params[a.off_hw[trunk] + d * h1 + k] : 0.f;
     }
     if (tid < H) {
-        B1[tid] = tid < a.h0 ? a.params[a.off_b1[trunk] + tid] : 0.f;
-        B2[tid] = tid < a.h1 ? a.params[a.off_b2[trunk] + tid] : 0.f;
+        B1[tid] = tid < h0 ? a.params[a.off_b1[trunk] + tid] : 0.f;
+        B2[tid] = tid < h1 ? a.params[a.off_b2[trunk] + tid] : 0.f;
     }
     if (tid < AMAX) HB[tid] = tid < AOUT ? a.params[a.off_hb[trunk] + tid] : 0.f;
     const int ty = tid >> 4, tx = tid & 15, hr = tid >> 2, hq = tid & 3;

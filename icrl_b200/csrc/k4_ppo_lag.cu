@@ -333,13 +333,20 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
     else if (tid < 128 + AOUT) { s_kind = 2; s_idx = tid - 128; }
     else if (tid >= 160 && tid < 160 + a.A && has_logstd) { s_kind = 3; s_idx = tid - 160; }
 
-    auto flat_w2 = [&](int j, int k) { return (j < a.h1 && k < a.h0) ? a.off_w2[trunk] + j * a.h0 + k : -1; };
-    auto flat_w1 = [&](int j, int k) { return (j < a.h0 && k < D) ? a.off_w1[trunk] + j * D + k : -1; };
-    auto flat_hw = [&](int d, int k) { return (d < AOUT && k < a.h1) ? a.off_hw[trunk] + d * a.h1 + k : -1; };
+    // flat index of an owned parameter, -1 for the padding of this CTA's trunk
+    auto flat_w2 = [&](int j, int k) {
+        const int h0 = a.h0[trunk];
+        return (j < a.h1[trunk] && k < h0) ? a.off_w2[trunk] + j * h0 + k : -1;
+    };
+    auto flat_w1 = [&](int j, int k) { return (j < a.h0[trunk] && k < D) ? a.off_w1[trunk] + j * D + k : -1; };
+    auto flat_hw = [&](int d, int k) {
+        const int h1 = a.h1[trunk];
+        return (d < AOUT && k < h1) ? a.off_hw[trunk] + d * h1 + k : -1;
+    };
     auto flat_scalar = [&]() {
         switch (s_kind) {
-            case 0: return s_idx < a.h0 ? a.off_b1[trunk] + s_idx : -1;
-            case 1: return s_idx < a.h1 ? a.off_b2[trunk] + s_idx : -1;
+            case 0: return s_idx < a.h0[trunk] ? a.off_b1[trunk] + s_idx : -1;
+            case 1: return s_idx < a.h1[trunk] ? a.off_b2[trunk] + s_idx : -1;
             case 2: return a.off_hb[trunk] + s_idx;
             case 3: return a.off_logstd + s_idx;
         }
@@ -1472,7 +1479,8 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
                 ac.inv_bc2_sqrt = adam_inv_bc2_sqrt;
                 ac.eps = (float)a.adam_eps;
                 ac.neg_step_size = adam_neg_step;
-                // padding entries (j >= h1, k >= h0 / D) keep g = m = v = 0 and therefore stay exactly 0
+                // padding entries of this CTA's trunk (j >= its h1, k >= its h0 / D) keep g = m = v = 0 and therefore stay
+                // exactly 0: their weights and biases are 0, so tanh(0) = 0 and every gradient into them is a product with 0
 #pragma unroll
                 for (int nt = 0; nt < NTW2; ++nt) {
                     float2* pa = reinterpret_cast<float2*>(W2 + oj * LDH + w2_k(nt));

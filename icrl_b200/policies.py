@@ -82,9 +82,11 @@ class ActorTwoCriticsPolicy:
         if len(net_arch) != 1 or not isinstance(net_arch[0], dict):
             raise NotImplementedError("shared policy layers (-sl) are not implemented; use separate pi/vf/cvf trunks")
         pi, vf, cvf = (list(net_arch[0].get(k, [])) for k in ("pi", "vf", "cvf"))
-        if not (pi == vf == cvf and len(pi) == 2 and max(pi) <= 64):
-            raise NotImplementedError(f"net_arch {net_arch}: the kernels support three identical two-layer trunks of "
-                                      "width <= 64 (the reference default is [64, 64])")
+        for key, sizes in zip(("pi", "vf", "cvf"), (pi, vf, cvf)):
+            if len(sizes) != 2 or not all(1 <= int(h) <= 64 for h in sizes):
+                raise NotImplementedError(f"net_arch {net_arch}: the {key} trunk {sizes} is not supported; the kernels "
+                                          "support two-layer pi / vf / cvf trunks of widths 1..64 each (the reference "
+                                          "default is [64, 64])")
         self.observation_space, self.action_space = observation_space, action_space
         self.net_arch, self.activation_fn, self.ortho_init = net_arch, activation_fn, ortho_init
         self.is_discrete = _is_discrete(action_space)
@@ -92,7 +94,7 @@ class ActorTwoCriticsPolicy:
         self.act_out = int(action_space.n) if self.is_discrete else int(np.prod(action_space.shape))
         if self.act_out > 16:
             raise NotImplementedError("more than 16 action dimensions")
-        self.hidden = (int(pi[0]), int(pi[1]))
+        self.trunk_hidden = tuple((int(t[0]), int(t[1])) for t in (pi, vf, cvf))   # {h0, h1} of pi, vf, cvf
         self.log_std_init = log_std_init
         if optimizer_kwargs is None:
             optimizer_kwargs = {"eps": 1e-5}                               # policies.py:357-361
@@ -142,7 +144,8 @@ class ActorTwoCriticsPolicy:
     def make_cfg(self, **kw) -> _lib.PpoCfg:
         cfg = _lib.PpoCfg()
         cfg.obs_dim, cfg.act_dim, cfg.is_discrete = self.obs_dim, self.act_out, int(self.is_discrete)
-        cfg.hidden[0], cfg.hidden[1] = self.hidden
+        for t, (h0, h1) in enumerate(self.trunk_hidden):
+            cfg.trunk_hidden[t][0], cfg.trunk_hidden[t][1] = h0, h1
         cfg.T = cfg.E = 1
         cfg.batch_size = cfg.n_epochs = 1
         g = getattr(self, "optimizer", None)

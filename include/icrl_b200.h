@@ -182,10 +182,11 @@ int icrl_dual_gae_host(const float* rewards, const float* reward_values, const f
  * nu * cost term, both value losses, entropy, backward, clip_grad_norm_, Adam -- for every minibatch of
  * every epoch in ONE persistent launch, with the per-epoch target_kl early stop evaluated on the device.
  *
- * Policy: three separate tanh MLP trunks obs -> hidden[0] -> hidden[1] (pi, vf, cvf; torch_layers.py:129-254)
- * and linear heads.  `params` / `adam_m` / `adam_v` are flat float32 device vectors in the reference's
- * parameters() order: [log_std (act_dim, continuous only)], then for pi, vf, cvf: W0 (h0 x obs_dim), b0,
- * W1 (h1 x h0), b1; then action_net W (act_out x h1), b; value_net W (1 x h1), b; cost_value_net W, b.
+ * Policy: three separate tanh MLP trunks obs -> h0 -> h1 (pi, vf, cvf; torch_layers.py:129-254), each with its own
+ * {h0, h1} (`trunk_hidden`, or `hidden` for all three), and linear heads on their own trunk's last layer.  `params` /
+ * `adam_m` / `adam_v` are flat float32 device vectors in the reference's parameters() order: [log_std (act_dim,
+ * continuous only)], then for each trunk t of pi, vf, cvf: W0 (h0[t] x obs_dim), b0, W1 (h1[t] x h0[t]), b1; then
+ * action_net W (act_out x h1[pi]), b; value_net W (1 x h1[vf]), b; cost_value_net W (1 x h1[cvf]), b.
  *
  * Rollout data are device arrays in the buffer's TIME-MAJOR layout [T, E, ...]; minibatch indices in
  * `perm` refer to the reference's env-major flattening (row = e*T + t, buffers.py:52-65,598-603) and are
@@ -211,6 +212,9 @@ typedef struct icrl_ppo_cfg {
     float nu;                               /* current penalty self.dual.nu().item() (ppo_lag.py:234) */
     double lr, adam_beta1, adam_beta2, adam_eps;
     int32_t max_steps;                      /* >0: stop after that many optimiser steps (bench sampling); 0 = all */
+    int32_t trunk_hidden[3][2];             /* {h0, h1} of the pi, vf and cvf trunks, each in 1..64; all zeros: every trunk
+                                               uses hidden[] (so zero-initialising callers keep the shared widths).  When
+                                               set, hidden[] is ignored.  Appended without an ABI version change. */
 } icrl_ppo_cfg;
 
 typedef struct icrl_ppo_data {
