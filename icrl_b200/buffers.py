@@ -137,9 +137,10 @@ class RolloutBufferWithCost:
             orig_h = self._d2h("relabel_orig_out", orig)
             costs_h = orig_h if costs is orig else self._d2h("relabel_costs_out", costs)
             th.cuda.current_stream().synchronize()
-            if vn is not None and vn.training:
+            if vn is not None:
                 state = state_h.numpy()
-                vn.cost_rms.mean, vn.cost_rms.var, vn.cost_rms.count = state[0], state[1], float(state[2])
+                if vn.training:
+                    vn.cost_rms.mean, vn.cost_rms.var, vn.cost_rms.count = state[0], state[1], float(state[2])
                 vn.cost_ret = state[3:].copy()
             self.orig_costs = orig_h.numpy().copy()
             self.costs = self.orig_costs if costs is orig else costs_h.numpy().copy()

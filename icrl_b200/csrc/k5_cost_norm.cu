@@ -16,7 +16,7 @@
 //     ->  normalise + store (parallel)
 //   Measured on B200 (tools/micro/fp64_bench.cu): DFMA/DADD/DMUL issue at 64 lanes/cycle/SM with 8.5-cycle latency, but
 //   float<->double conversions (F2F) run at ~16 lanes/cycle/SM with ~22-cycle latency, hence no conversion on a chain.
-//   E > 64: three launches --
+//   E > 64, or no training: three launches (without training: A, then C when norm_cost) --
 //   A  cost_ret_kernel    one thread per environment: ret <- ret * gamma + c[t], store, zero at episode ends   (T-serial)
 //   B  cost_rms_kernel    one CTA: per-step batch mean/var (parallel over t), then the Chan merge chain on thread 0
 //   C  cost_apply_kernel  c / sqrt(var_t + eps), clip, -> float32                                              (parallel)
@@ -28,7 +28,7 @@ namespace icrl {
 
 // numpy's pairwise summation (numpy/core/src/umath/loops_utils.h.src, @TYPE@_pairwise_sum) over f(a[i]).
 // The recursion for n > 128 is bounded at compile time (DEPTH levels, each a real call) so that the stack is sized
-// statically: DEPTH = 12 covers n <= 128 * 2^12 environments.
+// statically; pw_max_n(DEPTH) below is how many elements DEPTH levels cover.
 template <int DEPTH, class F>
 __device__ __noinline__ double np_pairwise_sum(const double* a, int n, F f) {
     if (n < 8) {
@@ -55,11 +55,21 @@ __device__ __noinline__ double np_pairwise_sum(const double* a, int n, F f) {
         n2 -= n2 % 8;
         return __dadd_rn(np_pairwise_sum<DEPTH - 1>(a, n2, f), np_pairwise_sum<DEPTH - 1>(a + n2, n - n2, f));
     } else {
-        return __longlong_as_double(0x7ff8000000000000LL);   // unreachable: E is validated on the host
+        return __longlong_as_double(0x7ff8000000000000LL);   // unreachable for n <= pw_max_n(DEPTH): see kMaxEnvs
     }
 }
-constexpr int kPwDepth = 12;
-constexpr int kMaxEnvs = 128 << kPwDepth;
+// The largest m such that every n <= m reaches blocks of at most 128 within `depth` splits.  numpy's split of
+// n = 16k + r (0 <= r < 16) is n2 = 8k, so the larger half is 8k + r and the halves are uneven: the first n whose larger
+// half exceeds p = pw_max_n(depth - 1) is p + 1 + 8 * ceil((p - 14) / 8), well below 128 * 2^depth (491 529 needs 13
+// levels, not 12).  Not monotone above that bound (256 needs one level, 249 two), hence "every n <= m".
+constexpr int pw_max_n(int depth) {
+    int m = 128;
+    for (int d = 0; d < depth; ++d) m += 8 * ((m - 14 + 7) / 8);
+    return m;
+}
+constexpr int kPwDepth = 13;
+constexpr int kMaxEnvs = 128 << 12;   // 524 288 environments per rollout
+static_assert(kMaxEnvs <= pw_max_n(kPwDepth), "np_pairwise_sum<kPwDepth> must cover every accepted E");
 
 // RunningMeanStd.update_from_moments, one step (shared by the fused and the three-launch paths).
 __device__ __forceinline__ void rms_step(double bm, double bv, double n, double& mean, double& var, double& count) {
@@ -88,16 +98,19 @@ __device__ __forceinline__ double div_known_rcp(double a, double b, double r) {
 __device__ __forceinline__ bool significand_all_ones(double b) {
     return (__double_as_longlong(b) & 0x000fffffffffffffLL) == 0x000fffffffffffffLL;
 }
-// A: discounted cost return per environment.  state = {mean, var, count, cost_ret[E]} (float64).
+// A: discounted cost return per environment.  state = {mean, var, count, cost_ret[E]} (float64).  Without training the
+// return is not accumulated but is still zeroed at episode ends, as VecNormalizeWithCost.step_wait does (ret_t unused).
 __global__ void cost_ret_kernel(const float* __restrict__ orig_costs, const float* __restrict__ dones,
-                                const uint8_t* __restrict__ last_dones, int T, int E, double gamma,
+                                const uint8_t* __restrict__ last_dones, int T, int E, double gamma, int training,
                                 double* __restrict__ state, double* __restrict__ ret_t) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= E) return;
     double ret = state[3 + e];
     for (int t = 0; t < T; ++t) {
-        ret = __dadd_rn(__dmul_rn(ret, gamma), (double)orig_costs[(size_t)t * E + e]);
-        ret_t[(size_t)t * E + e] = ret;
+        if (training) {
+            ret = __dadd_rn(__dmul_rn(ret, gamma), (double)orig_costs[(size_t)t * E + e]);
+            ret_t[(size_t)t * E + e] = ret;
+        }
         // `news` of step t is what the buffer stores as dones[t + 1] (on_policy_algorithm.py:406-415)
         const bool ended = (t + 1 < T) ? (dones[(size_t)(t + 1) * E + e] != 0.f) : (last_dones[e] != 0);
         if (ended) ret = 0.0;
@@ -424,11 +437,14 @@ extern "C" int icrl_cost_normalize(const float* orig_costs, const float* dones, 
     if (training) {
         if (int rc = device_scratch(SLOT_WORK3, ((size_t)total + 3 * (size_t)T) * sizeof(double), (void**)&scratch)) return rc;
         double *ret_t = scratch, *bmean = scratch + total, *bvar = bmean + T, *var_t = bvar + T;
-        cost_ret_kernel<<<(E + 63) / 64, 64, 0, st>>>(orig_costs, dones, last_dones, T, E, cost_gamma, state, ret_t);
+        cost_ret_kernel<<<(E + 63) / 64, 64, 0, st>>>(orig_costs, dones, last_dones, T, E, cost_gamma, 1, state, ret_t);
         ICRL_LAUNCH_CHECK();
         cost_rms_kernel<<<1, 1024, 0, st>>>(ret_t, T, E, state, bmean, bvar, var_t);
         ICRL_LAUNCH_CHECK();
         scratch = var_t;
+    } else {
+        cost_ret_kernel<<<(E + 63) / 64, 64, 0, st>>>(orig_costs, dones, last_dones, T, E, cost_gamma, 0, state, nullptr);
+        ICRL_LAUNCH_CHECK();
     }
     if (norm_cost) {
         const int blocks = (int)((total + 255) / 256 < (long long)sm_count() * 8 ? (total + 255) / 256 : (long long)sm_count() * 8);

@@ -303,9 +303,10 @@ int icrl_dual_update(float* state, const float* orig_costs, int64_t n, double al
  *   dones      [T, E] float32   buffer layout: dones[t] = episode ended at step t-1 (buffers.py add());
  *   last_dones [E]    uint8     episode ended at step T-1            -> `news` of step t = dones[t+1] / last_dones
  *   state      float64 [3 + E]  {cost_rms.mean, cost_rms.var, cost_rms.count, cost_ret[E]}, read and updated when
- *                               `training` (bit-exact with the numpy float64 arithmetic, pairwise sums included)
+ *                               `training` (bit-exact with the numpy float64 arithmetic, pairwise sums included);
+ *                               without `training` only cost_ret changes: zeroed where an episode ended
  *   costs      [T, E] float32   clip(orig / sqrt(var_after_step_t + epsilon), +-clip_cost) when `norm_cost`, else a copy
- * (may alias orig_costs). */
+ * (may alias orig_costs).  1 <= E <= 524288. */
 int icrl_cost_normalize(const float* orig_costs, const float* dones, const uint8_t* last_dones, int32_t T, int32_t E,
                         double cost_gamma, double epsilon, double clip_cost, int32_t norm_cost, int32_t training,
                         double* state, float* costs, void* stream);
