@@ -59,7 +59,7 @@ class PpoCfg(C.Structure):
         ("ent_coef", C.c_float), ("reward_vf_coef", C.c_float), ("cost_vf_coef", C.c_float),
         ("max_grad_norm", C.c_float), ("target_kl", C.c_float), ("nu", C.c_float),
         ("lr", C.c_double), ("adam_beta1", C.c_double), ("adam_beta2", C.c_double), ("adam_eps", C.c_double),
-        ("max_steps", C.c_int32), ("trunk_hidden", (C.c_int32 * 2) * 3),
+        ("max_steps", C.c_int32), ("trunk_hidden", (C.c_int32 * 2) * 3), ("n_shared", C.c_int32),
     ]
 
 

@@ -58,6 +58,7 @@ struct PpoArgs {
     float* wide_part;             // [3 trunks][ncl][F][256 threads]: every cluster's pair-summed gradient fragments
     float* wide_red;              // [3 trunks][F][256 threads]: the cluster-order sums
     unsigned int* wide_sync;      // [3 trunks] arrival counters of the grid-wide barriers (zeroed before every launch)
+    int n_shared;                 // leading layers shared by the three trunks (0, 1, 2): their off_* point at one tensor
 };
 constexpr int WIDE_SMAX = 6;      // floats a (cluster, half) reducer sums per step: F <= 2 * ncl * WIDE_SMAX
 constexpr int WIDE_MAXCTA = 192;  // CTAs of a wide launch (<= 32 clusters) addressable in the data-parallel receive buffer
@@ -68,16 +69,32 @@ constexpr int RSAG_MAXW = 20;     // 16-byte words per (rank, role, thread) slab
                                   // 2-rank broadcast),
                                   // overlaid on the same receive buffer (sequence numbers keep the two layouts apart)
 
+// Shared layers (n_shared >= 1) come first, as MlpExtractor.shared_net does in parameters(); every trunk's offsets of a
+// shared layer point at the one tensor, so code that reads a trunk through its offsets needs no other change.
 inline int ppo_fill_offsets(PpoArgs& a) {
     int o = 0;
     a.off_logstd = a.is_discrete ? -1 : 0;
     if (!a.is_discrete) o += a.A;
+    if (a.n_shared >= 1) {
+        const int w1 = o, b1 = w1 + a.h0[0] * a.D;
+        o = b1 + a.h0[0];
+        for (int t = 0; t < 3; ++t) { a.off_w1[t] = w1; a.off_b1[t] = b1; }
+    }
+    if (a.n_shared == 2) {
+        const int w2 = o, b2 = w2 + a.h1[0] * a.h0[0];
+        o = b2 + a.h1[0];
+        for (int t = 0; t < 3; ++t) { a.off_w2[t] = w2; a.off_b2[t] = b2; }
+    }
     for (int t = 0; t < 3; ++t) {
         const int h0 = a.h0[t], h1 = a.h1[t];
-        a.off_w1[t] = o; o += h0 * a.D;
-        a.off_b1[t] = o; o += h0;
-        a.off_w2[t] = o; o += h1 * h0;
-        a.off_b2[t] = o; o += h1;
+        if (a.n_shared < 1) {
+            a.off_w1[t] = o; o += h0 * a.D;
+            a.off_b1[t] = o; o += h0;
+        }
+        if (a.n_shared < 2) {
+            a.off_w2[t] = o; o += h1 * h0;
+            a.off_b2[t] = o; o += h1;
+        }
     }
     const int outs[3] = {a.A, 1, 1};
     for (int t = 0; t < 3; ++t) {
@@ -105,11 +122,20 @@ inline int ppo_make_args(const icrl_ppo_cfg* c, PpoArgs& a) {
                        "policy hidden sizes (%d, %d) must be in 1..%d (two hidden layers per trunk)", c->hidden[0],
                        c->hidden[1], H);
     }
+    ICRL_CHECK_ARG(c->n_shared >= 0 && c->n_shared <= 2, "n_shared = %d: 0, 1 or 2 shared layers (two layers per trunk)",
+                   c->n_shared);
     a.D = c->obs_dim; a.DP = ppo_ldx(c->obs_dim); a.KP = ppo_kp(c->obs_dim); a.A = c->act_dim; a.is_discrete = c->is_discrete;
     for (int t = 0; t < 3; ++t) {
         a.h0[t] = per_trunk ? c->trunk_hidden[t][0] : c->hidden[0];
         a.h1[t] = per_trunk ? c->trunk_hidden[t][1] : c->hidden[1];
     }
+    a.n_shared = c->n_shared;
+    ICRL_CHECK_ARG(a.n_shared < 1 || (a.h0[1] == a.h0[0] && a.h0[2] == a.h0[0]),
+                   "n_shared = %d: the shared first layer needs equal h0 in every trunk (pi %d, vf %d, cvf %d)", a.n_shared,
+                   a.h0[0], a.h0[1], a.h0[2]);
+    ICRL_CHECK_ARG(a.n_shared < 2 || (a.h1[1] == a.h1[0] && a.h1[2] == a.h1[0]),
+                   "n_shared = 2: the shared second layer needs equal h1 in every trunk (pi %d, vf %d, cvf %d)", a.h1[0],
+                   a.h1[1], a.h1[2]);
     a.T = c->T; a.E = c->E; a.N = c->T * c->E;
     a.B = c->batch_size > 0 ? c->batch_size : a.N;
     if (a.B > a.N && a.N > 0) a.B = a.N;

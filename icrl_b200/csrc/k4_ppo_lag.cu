@@ -46,6 +46,24 @@ __device__ __forceinline__ uint32_t cluster_nctarank() {
 __device__ __forceinline__ void cluster_sync_all() {
     asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
+// mbar_wait_bounded with cluster-scope acquire: the phase is completed by remote arrivals of peer CTAs
+__device__ __forceinline__ bool mbar_wait_bounded_cluster(uint64_t* bar, uint32_t parity, long long max_cycles) {
+    const long long t0 = clock64();
+    for (;;) {
+        uint32_t done;
+        asm volatile(
+            "{\n"
+            ".reg .pred p;\n"
+            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n"
+            "selp.u32 %0, 1, 0, p;\n"
+            "}\n"
+            : "=r"(done)
+            : "r"(smem_u32(bar)), "r"(parity)
+            : "memory");
+        if (done) return true;
+        if (clock64() - t0 > max_cycles) return false;
+    }
+}
 __device__ __forceinline__ void st_remote_f32(float* local_ptr, uint32_t rank, float v) {
     uint32_t a = smem_u32(local_ptr), ra;
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(a), "r"(rank));
@@ -62,9 +80,11 @@ constexpr int NTW2 = 4;        // n-tiles of a 64 x 64 output per warp (warp til
 
 // ---------------------------------------------------------------- shared memory carve-up (float offsets)
 struct PpoSmem {
-    int w1, w2, b1, b2, hw, hb, logstd, sig, x, h1, h2, dh, rowf, dmean, act, mu, part, bar, scratch, tacc, xch, pay, total_bytes;
+    int w1, w2, b1, b2, hw, hb, logstd, sig, x, h1, h2, dh, rowf, dmean, act, mu, part, bar, scratch, tacc, xch, pay, shr, shbar,
+        total_bytes;
 };
-__host__ __device__ inline PpoSmem ppo_smem_layout(int LDX, int NP) {
+// shared: the launch trains shared trunk layers and needs the activation-gradient exchange's receive tiles and barriers
+__host__ __device__ inline PpoSmem ppo_smem_layout(int LDX, int NP, bool shared = false) {
     PpoSmem s;
     int o = 0;
     s.w1 = o; o += H * LDX;          // W1[j][k], row stride LDX
@@ -89,6 +109,8 @@ __host__ __device__ inline PpoSmem ppo_smem_layout(int LDX, int NP) {
     s.tacc = o; o += 40;             // per-phase cycle counters of thread 0 (ICRL_PPO_TIMING): 20 x 8 bytes
     s.xch = o; o += 2 * 8 * 2;       // [parity][cluster rank][{sumsq, stop}]
     s.pay = o; o += NP * NTT;        // the partner CTA's gradient fragments land here (DSMEM stores)
+    s.shr = o; o += shared ? 2 * RBH * H : 0;   // the two other trunks' [RBH][H] activation-gradient tiles (DSMEM stores)
+    s.shbar = o; o += shared ? 4 : 0;           // two 8-byte mbarriers: tiles received, own tiles consumed by both peers
     s.total_bytes = o * 4;
     return s;
 }
@@ -273,7 +295,13 @@ struct TimingCounters<false> {
 // gradients meet in global memory (L2): write -> grid barrier -> each (cluster, half) sums its few floats over all clusters in
 // cluster order (and, data parallel, exchanges that slice with the peer GPUs' same reducer over NVLink) -> grid barrier ->
 // everybody reads the totals.  All replicas then apply the identical clip + Adam update, so they never diverge.
-template <int NT1, bool DIST, bool WIDE, bool TIMED>
+// SHARED (a.n_shared = 1 or 2 leading layers shared by the three trunks, MlpExtractor.shared_net; single GPU only): every
+// trunk keeps a replica of the shared layers and recomputes them on its rows, which are the same rows as the other trunks'
+// CTAs of the same half.  At the top of the shared part (dH1 with one shared layer, dH2 with two) the three CTAs of a half
+// swap their activation-gradient tiles through DSMEM and each adds the three in the fixed order (pi + vf) + cvf, so every
+// layer below back-propagates the same bits in all three trunks: the replicas get identical gradients, moments and updates
+// without any weight-gradient exchange.  Only the pi CTAs count the shared gradients in the norm and write them back.
+template <int NT1, bool DIST, bool WIDE, bool TIMED, bool SHARED = false>
 #ifdef ICRL_K4_MAXREG       // A/B builds (tools/build_variants.sh): an explicit register cap instead of the launch bounds
 #define ICRL_K4_BOUNDS __maxnreg__(ICRL_K4_MAXREG)
 #else
@@ -297,7 +325,7 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
     // bytes a CTA receives per step: every thread's groups, except the last one ({kl, entropy} sums), which only the threads
     // that own loss partials (hq == 0: every 8th) send
     constexpr int PAY_BYTES = (PAY_V4 - 1) * NTT * 16 + (NTT / 8) * 16;
-    const PpoSmem L = ppo_smem_layout(LDX, NP);
+    const PpoSmem L = ppo_smem_layout(LDX, NP, SHARED);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int crank = (int)cluster_ctarank();       // cluster rank: trunk = crank / 2 (0 pi, 1 vf, 2 cvf), half = crank % 2
     const int ncta = (int)cluster_nctarank();
@@ -306,6 +334,9 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
     const int trunk = working ? role : 0;
     const int AOUT = (role == 0) ? a.A : 1;
     const bool has_logstd = (role == 0) && !a.is_discrete;
+    // this CTA counts (norm) and writes back layer 1 / layer 2 of its trunk: a shared layer belongs to the pi CTAs
+    const bool own_l1 = !SHARED || role == 0;
+    const bool own_l2 = !SHARED || role == 0 || a.n_shared < 2;
 
     float* W1 = sm + L.w1; float* W2 = sm + L.w2;
     float* B1 = sm + L.b1; float* B2 = sm + L.b2; float* HW = sm + L.hw; float* HB = sm + L.hb;
@@ -420,6 +451,11 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
         mbar_init(&BAR[1], 1);
         mbar_init(&BAR[2], 1);     // pair exchange: armed by thread 0 every step, completed by the partner's st.async bytes
         mbar_init(&BAR[3], 1);     // norm exchange: completed by one 8-byte st.async from each CTA of the cluster
+        if constexpr (SHARED) {
+            uint64_t* SB = reinterpret_cast<uint64_t*>(sm + L.shbar);
+            mbar_init(&SB[0], 1);  // tiles received: armed by thread 0 every chunk, completed by the two peers' st.async bytes
+            mbar_init(&SB[1], 2);  // own tile consumed: one remote arrival from each of the two peers per chunk
+        }
         fence_mbar_init();
     }
     __syncthreads();
@@ -454,6 +490,60 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
         bulk_g2s(X + buf * RBH * LDX, a.xs + p * LDX, xb, &BAR[buf]);
         bulk_g2s(ROWF + buf * RBH * 8, a.ss + p * 8, sb, &BAR[buf]);
         if (role == 0) bulk_g2s(ACT + buf * RBH * AMAX, a.as + p * AP, ab, &BAR[buf]);
+    };
+
+    // ---- shared trunk layers: swap this chunk's activation-gradient tile T ([RBH][LDH]) with the CTAs of the same half of the
+    // other two trunks (the same rows) and replace it by the sum of the three in trunk order, identical bits in every trunk.
+    // One receive tile per peer: two per peer do not fit beside the NT1 = 8 layout (200.3 + 32 KB > 227 KB).  So a CTA sends
+    // its tile of chunk qx only after both peers have consumed the one of chunk qx - 1: each CTA arrives on both peers'
+    // "consumed" mbarrier after its sum and waits on its own before it sends.
+    auto share_tile = [&](float* T, int qx) {
+        if constexpr (SHARED) {
+            uint64_t* SB = reinterpret_cast<uint64_t*>(sm + L.shbar);
+            float* RX = sm + L.shr;
+            if (qx > 0 && *(volatile float*)&XCH[31] == 0.f &&
+                !mbar_wait_bounded_cluster(&SB[1], (uint32_t)((qx - 1) & 1), 2000000000LL))
+                XCH[31] = 1.f;
+            float4 mine[2];                                   // float4 groups i = tid, tid + 256 of the 32 x 64 tile
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+                const int i = tid + u * NTT;
+                mine[u] = *reinterpret_cast<const float4*>(T + (i >> 4) * LDH + 4 * (i & 15));
+            }
+#pragma unroll
+            for (int pp = 1; pp < 3; ++pp) {
+                const int prole = (role + pp) % 3;
+                const uint32_t prank = (uint32_t)(2 * prole + half);
+                const int slot = role - (role > prole ? 1 : 0);   // a receiver's two slots hold the other trunks in trunk order
+                uint32_t rx, rb;
+                asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rx) : "r"(smem_u32(RX + slot * RBH * H)), "r"(prank));
+                asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rb) : "r"(smem_u32(&SB[0])), "r"(prank));
+#pragma unroll
+                for (int u = 0; u < 2; ++u)
+                    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.f32 [%0], {%1, %2, %3, %4}, [%5];" ::"r"(
+                                     rx + (uint32_t)((tid + u * NTT) * 16)),
+                                 "f"(mine[u].x), "f"(mine[u].y), "f"(mine[u].z), "f"(mine[u].w), "r"(rb) : "memory");
+            }
+            if (*(volatile float*)&XCH[31] == 0.f && !mbar_wait_bounded(&SB[0], (uint32_t)(qx & 1), 2000000000LL)) XCH[31] = 1.f;
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+                const int i = tid + u * NTT;
+                const float4 x = *reinterpret_cast<const float4*>(RX + 4 * i);
+                const float4 y = *reinterpret_cast<const float4*>(RX + RBH * H + 4 * i);
+                const float4 t0 = role == 0 ? mine[u] : x;
+                const float4 t1 = role == 0 ? x : role == 1 ? mine[u] : y;
+                const float4 t2 = role == 2 ? mine[u] : y;
+                *reinterpret_cast<float4*>(T + (i >> 4) * LDH + 4 * (i & 15)) =
+                    make_float4((t0.x + t1.x) + t2.x, (t0.y + t1.y) + t2.y, (t0.z + t1.z) + t2.z, (t0.w + t1.w) + t2.w);
+            }
+            __syncthreads();          // the sum is complete in T, and no thread of this CTA reads its slots any more
+            if (tid < 2) {            // thread p tells peer p that its tile of this chunk has been consumed
+                uint32_t rb;
+                asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rb)
+                             : "r"(smem_u32(&SB[1])), "r"((uint32_t)(2 * ((role + 1 + tid) % 3) + half)));
+                asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(rb) : "memory");
+            }
+        }
     };
 
     Cursor cur = cur_skip_empty(Cursor{0, 0, 0});
@@ -542,6 +632,9 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
                         // phase cannot complete without this arrival).
                         mbar_expect_tx(&BAR[2], (uint32_t)PAY_BYTES);
                         mbar_expect_tx(&BAR[3], (uint32_t)(NCTA * 8));
+                    }
+                    if constexpr (SHARED) {   // this chunk's shared-layer tiles from the two peers (see share_tile)
+                        if (tid == 0) mbar_expect_tx(reinterpret_cast<uint64_t*>(sm + L.shbar), (uint32_t)(2 * RBH * H * 4));
                     }
                     ICRL_MARK(0)
                     {
@@ -833,6 +926,7 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
                     ICRL_MARK(15)
                     __syncthreads();
                     ICRL_MARK(5)
+                    if (SHARED && a.n_shared == 2) share_tile(DH, q);     // dH2pre of the three heads -> their sum
                     if (hd < AOUT) {
                         const float4 v = *reinterpret_cast<const float4*>(PART + hd * LDH + 4 * hk4);
                         g_hw[0] += v.x; g_hw[1] += v.y; g_hw[2] += v.z; g_hw[3] += v.w;
@@ -871,6 +965,7 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
                     }
                     __syncthreads();
                     ICRL_MARK(6)
+                    if (SHARED && a.n_shared == 1) share_tile(H2, q);     // dH1pre of the three trunks -> their sum
                     // ---- dW1[j][k] += sum_r dH1pre[r][j] X[r][k] ; db1
                     // every warp group has NT1 n-tiles inside the (zero padded) row when round16(D) == 16 NT1 -- true for all the
                     // named workloads; otherwise the last tile of the second group is skipped by the guarded variant
@@ -923,15 +1018,31 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
                 if (working) {
 #pragma unroll
                     for (int i = 0; i < 4; ++i) q2 = fmaf(g_hw[i], g_hw[i], q2);
+                    if constexpr (SHARED) {      // a shared layer's gradient counts once: in the pi CTAs' sums
+                        if (own_l2) {
 #pragma unroll
-                    for (int i = 0; i < NTW2; ++i)
+                            for (int i = 0; i < NTW2; ++i)
 #pragma unroll
-                        for (int c = 0; c < 4; ++c) q2 = fmaf(g_w2[i][c], g_w2[i][c], q2);
+                                for (int c = 0; c < 4; ++c) q2 = fmaf(g_w2[i][c], g_w2[i][c], q2);
+                        }
+                        if (own_l1) {
 #pragma unroll
-                    for (int i = 0; i < NT1; ++i)
+                            for (int i = 0; i < NT1; ++i)
 #pragma unroll
-                        for (int c = 0; c < 4; ++c) q2 = fmaf(g_w1[i][c], g_w1[i][c], q2);
-                    q2 = fmaf(g_s, g_s, q2);
+                                for (int c = 0; c < 4; ++c) q2 = fmaf(g_w1[i][c], g_w1[i][c], q2);
+                        }
+                        if ((s_kind != 0 || own_l1) && (s_kind != 1 || own_l2)) q2 = fmaf(g_s, g_s, q2);
+                    } else {
+#pragma unroll
+                        for (int i = 0; i < NTW2; ++i)
+#pragma unroll
+                            for (int c = 0; c < 4; ++c) q2 = fmaf(g_w2[i][c], g_w2[i][c], q2);
+#pragma unroll
+                        for (int i = 0; i < NT1; ++i)
+#pragma unroll
+                            for (int c = 0; c < 4; ++c) q2 = fmaf(g_w1[i][c], g_w1[i][c], q2);
+                        q2 = fmaf(g_s, g_s, q2);
+                    }
                 }
                 return q2;
             };
@@ -1541,14 +1652,14 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
         for (int nt = 0; nt < NTW2; ++nt)
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
-                const int j = frag_j(c), k = w2_k(nt) + frag_dk(c), f = flat_w2(j, k);
+                const int j = frag_j(c), k = w2_k(nt) + frag_dk(c), f = (SHARED && !own_l2) ? -1 : flat_w2(j, k);
                 if (f >= 0) { a.params[f] = W2[j * LDH + k]; a.adam_m[f] = m_w2[nt][c]; a.adam_v[f] = v_w2[nt][c]; }
             }
 #pragma unroll
         for (int i = 0; i < NT1; ++i)
 #pragma unroll
             for (int c = 0; c < 4; ++c) {
-                const int j = frag_j(c), k = w1_k(i) + frag_dk(c), f = flat_w1(j, k);
+                const int j = frag_j(c), k = w1_k(i) + frag_dk(c), f = (SHARED && !own_l1) ? -1 : flat_w1(j, k);
                 if (f >= 0) { a.params[f] = W1[j * LDX + k]; a.adam_m[f] = m_w1[i][c]; a.adam_v[f] = v_w1[i][c]; }
             }
 #pragma unroll
@@ -1556,7 +1667,7 @@ __global__ void ICRL_K4_BOUNDS ppo_train_kernel(const __grid_constant__ PpoArgs 
             const int f = flat_hw(hd, 4 * hk4 + kk);
             if (f >= 0) { a.params[f] = HW[hd * WA_LD + 4 * hk4 + kk]; a.adam_m[f] = m_hw[kk]; a.adam_v[f] = v_hw[kk]; }
         }
-        const int f = flat_scalar();
+        const int f = (SHARED && ((s_kind == 0 && !own_l1) || (s_kind == 1 && !own_l2))) ? -1 : flat_scalar();
         if (f >= 0) {
             const float* slot = s_kind == 0 ? &B1[s_idx] : s_kind == 1 ? &B2[s_idx] : s_kind == 2 ? &HB[s_idx] : &LOGSTD[s_idx];
             a.params[f] = *slot; a.adam_m[f] = m_s; a.adam_v[f] = v_s;
@@ -1589,7 +1700,11 @@ static int launch_cfg(const PpoArgs& a, cudaStream_t st, int n_clusters, cudaLau
     else
         kern = WIDE ? (a.world > 1 ? ppo_train_kernel<NT1, true, true, false> : ppo_train_kernel<NT1, false, true, false>)
                     : (a.world > 1 ? ppo_train_kernel<NT1, true, false, false> : ppo_train_kernel<NT1, false, false, false>);
-    const PpoSmem L = ppo_smem_layout(a.DP, ppo_pay_floats<NT1>());
+    // shared trunk layers: separate instantiations, so the kernels of separate trunks stay as they are (single GPU, no
+    // phase timing: the host refuses world > 1 and does not ask for timing with n_shared > 0)
+    if (a.n_shared > 0)
+        kern = WIDE ? ppo_train_kernel<NT1, false, true, false, true> : ppo_train_kernel<NT1, false, false, false, true>;
+    const PpoSmem L = ppo_smem_layout(a.DP, ppo_pay_floats<NT1>(), a.n_shared > 0);
     if (L.total_bytes > 227 * 1024) {
         set_error("obs_dim %d needs %d bytes of shared memory (> 227 KB)", a.D, L.total_bytes);
         return ICRL_EUNSUPPORTED;
@@ -1717,6 +1832,9 @@ static int ppo_train_impl(const icrl_ppo_cfg* cfg, const icrl_ppo_data* data, fl
     if (dist) {
         ICRL_CHECK_ARG(dist->world >= 1 && dist->world <= ICRL_PPO_MAX_RANKS && dist->rank >= 0 && dist->rank < dist->world,
                        "bad rank/world (%d/%d)", dist->rank, dist->world);
+        ICRL_CHECK_ARG(dist->world == 1 || a.n_shared == 0,
+                       "shared policy layers (n_shared = %d) are not supported in data-parallel training (world %d)",
+                       a.n_shared, dist->world);
         a.rank = dist->rank; a.world = dist->world; a.flag_base = dist->flag_base; a.advsums = dist->advsums;
         for (int r = 0; r < dist->world; ++r) {
             ICRL_CHECK_ARG(dist->world == 1 || (dist->recv[r] && dist->flags[r]), "peer buffer %d is NULL", r);
@@ -1754,7 +1872,7 @@ static int ppo_train_impl(const icrl_ppo_cfg* cfg, const icrl_ppo_data* data, fl
         return ICRL_EUNSUPPORTED;
     }
     static unsigned long long* timing_dev = nullptr;
-    const bool want_timing = getenv("ICRL_PPO_TIMING") != nullptr;
+    const bool want_timing = getenv("ICRL_PPO_TIMING") != nullptr && a.n_shared == 0;   // (no timed shared-layer kernel)
     if (want_timing && !timing_dev) cudaMalloc(&timing_dev, 128 * sizeof(unsigned long long));
     a.timing = want_timing ? timing_dev : nullptr;
     auto print_timing = [&](double steps) { ppo_print_timing(timing_dev, st, steps); };

@@ -1,5 +1,6 @@
 """ActorTwoCriticsPolicy -- host-side mirror of stable_baselines3/common/policies.py:598-779 (MlpPolicy flavour:
-FlattenExtractor, three separate tanh MLP trunks pi/vf/cvf, DiagGaussian or Categorical head).
+FlattenExtractor, three tanh MLP trunks pi/vf/cvf of two layers each, the first or both of them optionally shared
+(MlpExtractor.shared_net), DiagGaussian or Categorical head).
 
 Parameters and Adam moments live in flat float32 device tensors in the reference's `parameters()` order; the CUDA
 kernels (K4 train step, policy forward) read and update them in place.  A CPU `nn.Module` skeleton with the
@@ -23,29 +24,34 @@ from .spaces import is_discrete as _is_discrete
 
 
 class _MlpExtractorShape(nn.Module):
-    """Module skeleton with torch_layers.py:129-254's creation order (pi, vf, cvf layers interleaved) and names."""
+    """Module skeleton with torch_layers.py:129-254's creation order (shared layers, then pi, vf, cvf layers interleaved)
+    and names; a trunk without private layers takes the last shared width as its latent dimension."""
 
-    def __init__(self, feature_dim, pi, vf, cvf, activation_fn):
+    def __init__(self, feature_dim, shared, pi, vf, cvf, activation_fn):
         super().__init__()
+        shared_net, last_shared = [], feature_dim
+        for size in shared:
+            shared_net += [nn.Linear(last_shared, size), activation_fn()]
+            last_shared = size
         nets = {"policy_net": [], "value_net": [], "cost_value_net": []}
-        last = {k: feature_dim for k in nets}
+        last = {k: last_shared for k in nets}
         for sizes in zip_longest(pi, vf, cvf):
             for key, size in zip(nets, sizes):
                 if size is not None:
                     nets[key] += [nn.Linear(last[key], size), activation_fn()]
                     last[key] = size
         self.latent_dim_pi, self.latent_dim_vf, self.latent_dim_cvf = (last[k] for k in nets)
-        self.shared_net = nn.Sequential()
+        self.shared_net = nn.Sequential(*shared_net)
         self.policy_net = nn.Sequential(*nets["policy_net"])
         self.value_net = nn.Sequential(*nets["value_net"])
         self.cost_value_net = nn.Sequential(*nets["cost_value_net"])
 
 
 class _PolicyShape(nn.Module):
-    def __init__(self, obs_dim, act_out, discrete, pi, vf, cvf, activation_fn, log_std_init, ortho_init):
+    def __init__(self, obs_dim, act_out, discrete, pi, vf, cvf, activation_fn, log_std_init, ortho_init, shared=()):
         super().__init__()
         self.features_extractor = nn.Flatten()
-        self.mlp_extractor = _MlpExtractorShape(obs_dim, pi, vf, cvf, activation_fn)
+        self.mlp_extractor = _MlpExtractorShape(obs_dim, shared, pi, vf, cvf, activation_fn)
         self.action_net = nn.Linear(self.mlp_extractor.latent_dim_pi, act_out)
         if not discrete:
             self.log_std = nn.Parameter(th.ones(act_out) * log_std_init, requires_grad=True)
@@ -64,6 +70,39 @@ class _PolicyShape(nn.Module):
             module.bias.data.fill_(0.0)
 
 
+def _trunks(net_arch):
+    """net_arch -> (shared widths, pi, vf, cvf private widths, effective (h0, h1) of pi, vf, cvf).  The kernels train two
+    tanh layers of width 1..64 under every head: separate trunks [dict(pi=[a, b], vf=[c, d], cvf=[e, f])], one shared
+    layer [s, dict(pi=[p], vf=[v], cvf=[c])], or one shared trunk [s0, s1] (a dict there may only hold empty lists)."""
+    shared = []
+    for layer in net_arch:
+        if isinstance(layer, dict):
+            break
+        shared.append(layer)
+    rest = net_arch[len(shared):]
+    if len(rest) > 1 or (not shared and len(rest) != 1):
+        raise NotImplementedError(f"net_arch {net_arch}: expected shared layer widths followed by at most one dict of "
+                                  "pi / vf / cvf layers")
+    pi, vf, cvf = (list(rest[0].get(k, [])) if rest else [] for k in ("pi", "vf", "cvf"))
+    if not shared:
+        for key, sizes in zip(("pi", "vf", "cvf"), (pi, vf, cvf)):
+            if len(sizes) != 2 or not all(1 <= int(h) <= 64 for h in sizes):
+                raise NotImplementedError(f"net_arch {net_arch}: the {key} trunk {sizes} is not supported; the kernels "
+                                          "support two-layer pi / vf / cvf trunks of widths 1..64 each (the reference "
+                                          "default is [64, 64])")
+        return [], pi, vf, cvf, tuple((int(t[0]), int(t[1])) for t in (pi, vf, cvf))
+    if len(shared) > 2 or not all(isinstance(h, int) and 1 <= h <= 64 for h in shared):
+        raise NotImplementedError(f"net_arch {net_arch}: the shared layers {shared} are not supported; the kernels "
+                                  "support one or two shared layers of widths 1..64")
+    for key, sizes in zip(("pi", "vf", "cvf"), (pi, vf, cvf)):
+        if len(shared) + len(sizes) != 2 or not all(1 <= int(h) <= 64 for h in sizes):
+            raise NotImplementedError(f"net_arch {net_arch}: the {key} trunk, shared {shared} + private {sizes}, is not "
+                                      "supported; the kernels support two tanh layers of widths 1..64 under every head "
+                                      "(-sl s -pl p -rvl v -cvl c, or -sl s0 s1 with no private layers)")
+    effective = tuple((int(shared[0]), int(([*shared[1:], *sizes])[0])) for sizes in (pi, vf, cvf))
+    return [int(h) for h in shared], pi, vf, cvf, effective
+
+
 class ActorTwoCriticsPolicy:
     def __init__(self, observation_space, action_space, lr_schedule: Callable[[float], float],
                  net_arch: Optional[List] = None, activation_fn=nn.Tanh, ortho_init: bool = True, use_sde: bool = False,
@@ -79,14 +118,7 @@ class ActorTwoCriticsPolicy:
             raise NotImplementedError("icrl_b200 implements the reference's optimiser (Adam) only")
         if net_arch is None:
             net_arch = [dict(pi=[64, 64], vf=[64, 64], cvf=[64, 64])]
-        if len(net_arch) != 1 or not isinstance(net_arch[0], dict):
-            raise NotImplementedError("shared policy layers (-sl) are not implemented; use separate pi/vf/cvf trunks")
-        pi, vf, cvf = (list(net_arch[0].get(k, [])) for k in ("pi", "vf", "cvf"))
-        for key, sizes in zip(("pi", "vf", "cvf"), (pi, vf, cvf)):
-            if len(sizes) != 2 or not all(1 <= int(h) <= 64 for h in sizes):
-                raise NotImplementedError(f"net_arch {net_arch}: the {key} trunk {sizes} is not supported; the kernels "
-                                          "support two-layer pi / vf / cvf trunks of widths 1..64 each (the reference "
-                                          "default is [64, 64])")
+        shared, pi, vf, cvf, trunk_hidden = _trunks(net_arch)
         self.observation_space, self.action_space = observation_space, action_space
         self.net_arch, self.activation_fn, self.ortho_init = net_arch, activation_fn, ortho_init
         self.is_discrete = _is_discrete(action_space)
@@ -94,14 +126,15 @@ class ActorTwoCriticsPolicy:
         self.act_out = int(action_space.n) if self.is_discrete else int(np.prod(action_space.shape))
         if self.act_out > 16:
             raise NotImplementedError("more than 16 action dimensions")
-        self.trunk_hidden = tuple((int(t[0]), int(t[1])) for t in (pi, vf, cvf))   # {h0, h1} of pi, vf, cvf
+        self.trunk_hidden = trunk_hidden      # effective {h0, h1} of pi, vf, cvf (shared layers included)
+        self.n_shared = len(shared)           # leading layers the three trunks share
         self.log_std_init = log_std_init
         if optimizer_kwargs is None:
             optimizer_kwargs = {"eps": 1e-5}                               # policies.py:357-361
         self.optimizer_class, self.optimizer_kwargs = optimizer_class, optimizer_kwargs
         self.device = resolve_device(device)
         self._shape = _PolicyShape(self.obs_dim, self.act_out, self.is_discrete, pi, vf, cvf, activation_fn,
-                                   log_std_init, ortho_init)
+                                   log_std_init, ortho_init, shared)
         self._slices, off = [], 0
         for _, p in self._shape.named_parameters():
             self._slices.append((off, tuple(p.shape)))
@@ -146,6 +179,7 @@ class ActorTwoCriticsPolicy:
         cfg.obs_dim, cfg.act_dim, cfg.is_discrete = self.obs_dim, self.act_out, int(self.is_discrete)
         for t, (h0, h1) in enumerate(self.trunk_hidden):
             cfg.trunk_hidden[t][0], cfg.trunk_hidden[t][1] = h0, h1
+        cfg.n_shared = self.n_shared
         cfg.T = cfg.E = 1
         cfg.batch_size = cfg.n_epochs = 1
         g = getattr(self, "optimizer", None)

@@ -199,6 +199,10 @@ class PPOLagrangian:
         if comm is None:
             if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size() == 1:
                 return self
+        if self.policy.n_shared:
+            raise NotImplementedError(f"data-parallel training of shared policy layers (net_arch "
+                                      f"{self.policy.net_arch}) is not implemented")
+        if comm is None:
             from .distributed import PpoComm
             with th.cuda.device(self.device):
                 comm = PpoComm()
@@ -574,7 +578,8 @@ class PPOLagrangian:
         def plain(k, default=None):
             v = data.get(k, default)
             return default if isinstance(v, dict) and ":serialized:" in v else v
-        obs_dim = sd["mlp_extractor.policy_net.0.weight"].shape[1]
+        first = next(k for k in ("mlp_extractor.shared_net.0.weight", "mlp_extractor.policy_net.0.weight") if k in sd)
+        obs_dim = sd[first].shape[1]
         act_out = sd["action_net.weight"].shape[0]
         if env is not None:
             osp, asp = env.observation_space, env.action_space

@@ -186,7 +186,9 @@ int icrl_dual_gae_host(const float* rewards, const float* reward_values, const f
  * {h0, h1} (`trunk_hidden`, or `hidden` for all three), and linear heads on their own trunk's last layer.  `params` /
  * `adam_m` / `adam_v` are flat float32 device vectors in the reference's parameters() order: [log_std (act_dim,
  * continuous only)], then for each trunk t of pi, vf, cvf: W0 (h0[t] x obs_dim), b0, W1 (h1[t] x h0[t]), b1; then
- * action_net W (act_out x h1[pi]), b; value_net W (1 x h1[vf]), b; cost_value_net W (1 x h1[cvf]), b.
+ * action_net W (act_out x h1[pi]), b; value_net W (1 x h1[vf]), b; cost_value_net W (1 x h1[cvf]), b.  With `n_shared`
+ * > 0 the first or both layers are one tensor shared by the three trunks (MlpExtractor.shared_net) and come first, see
+ * icrl_ppo_cfg.n_shared.
  *
  * Rollout data are device arrays in the buffer's TIME-MAJOR layout [T, E, ...]; minibatch indices in
  * `perm` refer to the reference's env-major flattening (row = e*T + t, buffers.py:52-65,598-603) and are
@@ -215,6 +217,17 @@ typedef struct icrl_ppo_cfg {
     int32_t trunk_hidden[3][2];             /* {h0, h1} of the pi, vf and cvf trunks, each in 1..64; all zeros: every trunk
                                                uses hidden[] (so zero-initialising callers keep the shared widths).  When
                                                set, hidden[] is ignored.  Appended without an ABI version change. */
+    int32_t n_shared;                       /* leading layers the three trunks share (MlpExtractor.shared_net, the
+                                               reference's -sl): 0 separate trunks (zero-initialising callers), 1 a
+                                               shared obs -> h0 layer under private h0 -> h1[t] layers, 2 one obs -> h0
+                                               -> h1 trunk under all three heads.  The trunk widths above stay the
+                                               effective (h0, h1) of each trunk: n_shared >= 1 needs the three h0 equal,
+                                               n_shared == 2 the three h1 as well.  Layout of params / adam_m / adam_v:
+                                               [log_std], the shared layers (W0 (h0 x obs_dim), b0, and with n_shared == 2
+                                               W1 (h1 x h0), b1), the private layers W1 (h1[t] x h0), b1 of pi, vf and
+                                               cvf (n_shared == 1 only), then the heads.  Not supported by
+                                               icrl_ppo_train_dist with world > 1.  Appended without an ABI version
+                                               change. */
 } icrl_ppo_cfg;
 
 typedef struct icrl_ppo_data {

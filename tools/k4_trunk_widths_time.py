@@ -1,5 +1,5 @@
-"""K4 optimiser-step time per library build, alternating the builds, for policies with uniform 64-64 trunks and with
-per-trunk widths.
+"""K4 optimiser-step time per library build, alternating the builds, for policies with uniform 64-64 trunks, with
+per-trunk widths and with shared trunk layers.
 
 Shapes (one K4 launch each; us per optimiser step from CUDA events over `--launches` launches after one warm-up):
   hc            HalfCheetah: obs 18, 6 actions, batch 64, 10 epochs, one 10 240-row rollout (single cluster)
@@ -7,7 +7,13 @@ Shapes (one K4 launch each; us per optimiser step from CUDA events over `--launc
   ant_wide      Ant-shaped many-cluster launch: obs 113, 8 actions, 262 144 rows, batch 4 096, 2 epochs
   hc_mixed      the hc shape with pi (64, 64), vf (32, 32), cvf (16, 48); its 64-64 embedding is `hc`
   ant_mixed     the antwall shape with pi (64, 64), vf (64, 32), cvf (48, 64)
-The *_mixed shapes run only on builds that take per-trunk widths (`name=path+` below).
+  hc_sl1        the hc shape with net_arch [64, dict(pi=[64], vf=[32], cvf=[16])] (-sl 64); hc_sl1_sep: the same widths
+                as separate trunks, pi (64, 64), vf (64, 32), cvf (64, 16)
+  ant_sl1       the antwall shape (two chunks per step) with [64, dict(pi=[64], vf=[64], cvf=[48])]; ant_sl1_sep
+  hc_sl2        the hc shape with one trunk under all three heads, [64, 64]; its separate-trunk net is `hc`
+  ant_wide_sl1  the ant_wide shape (many clusters) with [64, dict(pi=[64], vf=[64], cvf=[64])]; its separate net is
+                `ant_wide`
+The *_mixed, *_sep and *_sl* shapes run only on builds that take per-trunk widths and shared layers (`name=path+`).
 
 Usage: python tools/k4_trunk_widths_time.py [--reps 5] [--launches 5] name=path/to/libicrl_b200.so[+] ...
   e.g. branch=icrl_b200/libicrl_b200.so+ parent=tools/_variants/parent.so
@@ -26,6 +32,12 @@ SHAPES = {   # obs_dim, actions, rows (T x E), batch, epochs, trunks
     "ant_wide": (113, 8, (2048, 128), 4096, 2, ((64, 64),) * 3),
     "hc_mixed": (18, 6, (2048, 5), 64, 10, ((64, 64), (32, 32), (16, 48))),
     "ant_mixed": (113, 8, (2048, 5), 128, 20, ((64, 64), (64, 32), (48, 64))),
+    "hc_sl1": (18, 6, (2048, 5), 64, 10, [64, dict(pi=[64], vf=[32], cvf=[16])]),   # a list: net_arch itself
+    "hc_sl1_sep": (18, 6, (2048, 5), 64, 10, ((64, 64), (64, 32), (64, 16))),
+    "ant_sl1": (113, 8, (2048, 5), 128, 20, [64, dict(pi=[64], vf=[64], cvf=[48])]),
+    "ant_sl1_sep": (113, 8, (2048, 5), 128, 20, ((64, 64), (64, 64), (64, 48))),
+    "hc_sl2": (18, 6, (2048, 5), 64, 10, [64, 64]),
+    "ant_wide_sl1": (113, 8, (2048, 128), 4096, 2, [64, dict(pi=[64], vf=[64], cvf=[64])]),
 }
 
 
@@ -47,12 +59,13 @@ def child(lib_path, mixed, launches):
     dev = th.device("cuda")
     out = {}
     for name, (D, A, (T, E), B, n_epochs, trunks) in SHAPES.items():
-        uniform = len(set(trunks)) == 1
+        uniform = isinstance(trunks, tuple) and len(set(trunks)) == 1
         if not uniform and not mixed:
             continue
         th.manual_seed(0)
+        net_arch = trunks if isinstance(trunks, list) else [dict(zip(("pi", "vf", "cvf"), (list(t) for t in trunks)))]
         pol = ActorTwoCriticsPolicy(Box(-1e9, 1e9, (D,)), Box(-1, 1, (A,)), lambda _: 3e-4, device=dev,
-                                    net_arch=[dict(zip(("pi", "vf", "cvf"), (list(t) for t in trunks)))])
+                                    net_arch=net_arch)
         n = T * E
         obs = th.randn(n, D, device=dev)
         acs = th.randn(n, A, device=dev)
@@ -118,7 +131,7 @@ def main(argv):
             v = sorted(r[shape] for r in runs[name] if shape in r)
             if v:
                 cells.append(f"{name} {v[len(v) // 2]:.2f} ({v[0]:.2f}..{v[-1]:.2f})")
-        print(f"  {shape:10s} " + "   ".join(cells))
+        print(f"  {shape:12s} " + "   ".join(cells))
 
 
 if __name__ == "__main__":
